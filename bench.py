@@ -163,6 +163,22 @@ class ClockSampler:
                 "power_w_max": max(pw) if pw else None, "reasons": reasons, "samples": len(sm)}
 
 
+def dump_sample(a, n=1 << 22):
+    """`a` flattened; past n entries, a fixed seeded sample of n of them (same indices for the same length)."""
+    a = np.asarray(a).ravel()
+    if a.size <= n:
+        return a
+    return a[np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))]
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy, float64 kept, everything else as float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
+
+
 def dist_setup(n_gpus):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -347,11 +363,13 @@ def run_ours(args, rank, local, world):
             self.i += 1
             return self.b[self.i % len(self.b)]
 
+    last = {}                                         # what the most recent step returned to its caller
+
     def one_step(loader):
         if train:
-            model.trainIteration(loader)
+            last["loss"] = model.trainIteration(loader)
         else:
-            eng.retrieve(loader.getTrainBatch(p), use_gt=True)
+            last["ranks"] = eng.retrieve(loader.getTrainBatch(p), use_gt=True)
 
     def timed(loader, steps, profile):
         barrier(world)
@@ -375,7 +393,7 @@ def run_ours(args, rank, local, world):
         sampler.start()
 
     if not train:                                     # ---- C5: ranker sweep
-        sweep = {}
+        sweep, outputs = {}, {}
         for Bs in cfg["sweep"]:
             host_b, dev_b = make_batches(Bs, n=2)
             dl, hl = Loader(dev_b), Loader(host_b)
@@ -385,6 +403,7 @@ def run_ours(args, rank, local, world):
             if rank == 0 and Bs == cfg["sweep"][0]:
                 sampler.mark_begin()
             ms, _, launches = timed(dl, args.steps, 0)
+            outputs["ranks_b%d" % Bs] = last["ranks"]
             ms_h, wall_h, _ = timed(hl, args.steps, 0)
             ms = max_over_ranks(ms, world)
             ms_h = max_over_ranks(max(ms_h, wall_h), world)
@@ -397,6 +416,8 @@ def run_ours(args, rank, local, world):
         clocks = sampler.stop() if rank == 0 else None
         if rank != 0:
             return
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         best = max(sweep, key=lambda k: sweep[k]["value"])
         line = {"metric": metric_name(args.config), "value": sweep[best]["value"], "unit": "QA-rounds/s", "n_gpus": world,
                 "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": sweep[best]["ms_per_step"],
@@ -429,6 +450,10 @@ def run_ours(args, rank, local, world):
     ms_dev, wall_dev, launches = timed(dev_loader, args.steps, 0 if args.ncu_range else 2)
     if args.ncu_range:
         eng.profiler_range(False)
+    if args.dump_outputs and rank == 0:         # replicas are identical after the all-reduce: rank 0 speaks for all
+        # the weights and gradients are 9-25 M entries per config: a sample of each keeps the dump under 64 MB
+        dump_outputs(args.dump_outputs, {"loss": np.float64([last["loss"]]), "weights": dump_sample(model.wrapperW.numpy()),
+                                         "gradients": dump_sample(model.wrapperdW.numpy())})
     stats_shared = {k: eng.kernel_stats(k) for k in LSTM_STEP_KEYS}
     ms_e2e, wall_e2e, _ = timed(host_loader, args.steps, 0)
     # Roofline pass: in the timed region above the option-LSTM kernels share the GPU with the encoder's concurrent
@@ -632,7 +657,11 @@ def main():
     ap.add_argument("--no-resident", action="store_true", help=argparse.SUPPRESS)      # accepted for old command lines
     ap.add_argument("--corpus-dialogs", type=int, default=256, help="dialogs in the synthetic resident corpus per rank")
     ap.add_argument("--ncu-range", action="store_true", help="bracket the timed steps with cudaProfilerStart/Stop")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (training: loss, and a "
+                    "seeded sample of the weights and gradients after it; C5: the ranks of each batch size) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
